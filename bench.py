@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- layouts/sec of the LayoutDM denoising loop (BASELINE.json metric) on N GPUs of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A "step" is one full pass of the hot path over one batch: `sample()` of B=1024 layouts per GPU through all T=100
@@ -11,6 +11,8 @@ the host-buffer C-ABI entry (ldm_sample_host: pinned-host inputs -> H2D -> loop 
 `roofline` = the dominant kernel against the measured bf16 tensor peak; `cpu_baseline` = the unmodified reference's
 `LayoutDM.sample` on the host cores (bounded sample; packaged by oracle/make_ref.py), `gpu_eager_baseline` = the same
 reference run eagerly on the GPU.  `--impl reference` times the CPU reference alone.
+`--dump-outputs DIR` writes what the last timed step returned (the final token ids, as float32) to DIR/ids.npy; weights
+and noise keys are fixed by the arguments, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -23,6 +25,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 REPO = os.path.dirname(os.path.abspath(__file__))
@@ -333,6 +336,20 @@ def other_configs(local):
     return out
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, ids):
+    """ids (layouts, S) -> path/ids.npy as float32 (token ids are exact there); above DUMP_LIMIT_BYTES a fixed, seeded
+    sample of layouts (rows kept in order) is written instead"""
+    os.makedirs(path, exist_ok=True)
+    a = ids.cpu().numpy().astype(np.float32)
+    max_rows = DUMP_LIMIT_BYTES // (a.shape[1] * a.itemsize)
+    if a.shape[0] > max_rows:
+        a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], max_rows, replace=False))]
+    np.save(os.path.join(path, "ids.npy"), a)
+
+
 # --------------------------------------------------------------------------------------------------------------
 def run_b200_arm(args, world, rank, local):
     from layoutdm_b200 import Engine, Vocab, timestep_plan
@@ -374,6 +391,8 @@ def run_b200_arm(args, world, rank, local):
         torch.cuda.synchronize(); barrier(world)
         ms_total = e0.elapsed_time(e1)
     launches = eng.launch_count - l0
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     ms_total = max_over_ranks(ms_total, world, dev)
     ms_step = ms_total / args.steps
     value = total / (ms_step * 1e-3)
@@ -455,7 +474,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the sub-records of BASELINE.json configs 0 / 2 / 3")
     ap.add_argument("--total-batch", type=int, default=0, help="strong scaling: this many layouts in total, split over the ranks")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the ids of the last timed step to DIR/ids.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the output of --impl b200")
     if args.impl == "reference":
         world, rank = int(os.environ.get("WORLD_SIZE", "1")), int(os.environ.get("RANK", "0"))
         run_reference_arm(args, world, rank)

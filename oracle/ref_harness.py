@@ -110,6 +110,37 @@ def synthetic_layouts(B: int, n_cat: int, seed: int = 0, max_elem: int = 25) -> 
     return FakeBatch(x, y, batch)
 
 
+def make_relation_batch(B, n_cat, seed, edge_ratio=0.3) -> FakeBatch:
+    """synthetic cond=relation batch built with the reference's own transforms (AddCanvasElement, AddRelationConstraints,
+    data/util.py:106-170): element 0 of every layout is the canvas, edges carry the relation labels"""
+    _setup_path()
+    from trainer.data.util import AddCanvasElement, AddRelationConstraints
+    g = torch.Generator().manual_seed(seed)
+    add_c, add_r = AddCanvasElement(), AddRelationConstraints(seed=seed, edge_ratio=edge_ratio)
+    xs, ys, bs, ei, ea = [], [], [], [], []
+    off = 0
+    for b in range(B):
+        n = int(torch.randint(1, 26, (1,), generator=g)) if b else 25
+        class D:
+            pass
+        d = D()
+        d.x = torch.rand(n, 4, generator=g) * torch.tensor([1.0, 1.0, 0.6, 0.6]) + torch.tensor([0.0, 0.0, 0.02, 0.02])
+        d.y = torch.randint(0, n_cat, (n,), generator=g)
+        d.attr = {"has_canvas_element": torch.tensor(False)}
+        d = add_c(d)
+        d.attr["has_canvas_element"] = True
+        d = add_r(d)
+        xs.append(d.x); ys.append(d.y); bs.append(torch.full((n + 1,), b))
+        if d.edge_index.numel():
+            ei.append(d.edge_index + off); ea.append(d.edge_attr)
+        off += n + 1
+    batch = FakeBatch(torch.cat(xs), torch.cat(ys), torch.cat(bs))
+    batch.edge_index = torch.cat(ei, dim=1) if ei else torch.zeros(2, 0, dtype=torch.long)
+    batch.edge_attr = torch.cat(ea) if ea else torch.zeros(0, dtype=torch.long)
+    batch.attr = {"has_canvas_element": True}
+    return batch
+
+
 @contextmanager
 def injected_multinomial(uniform_fn):
     """Replace torch.multinomial(probs, 1) by argmax(probs / -log(u)) with u supplied by the caller

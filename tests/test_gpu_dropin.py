@@ -110,7 +110,6 @@ def test_patched_model_relation_device_vs_reference_autograd_update():
     """cond = "relation" end to end on a live reference model: the device update kernel (default) against the reference's own
     autograd `update` running through the log-prob taps (relation_on_device = False), same noise key"""
     import random
-    from test_oracle_relation import make_relation_batch
     fx = Fixture("rico25_uncond_random")
     model, tok = patched(fx)
     fused = model.model.module._ldm_b200
@@ -118,7 +117,7 @@ def test_patched_model_relation_device_vs_reference_autograd_update():
     from trainer.helpers.task import get_cond
     random.seed(0); torch.manual_seed(0)
     B = 6
-    batch = make_relation_batch(B, fx.vocab.n_cat, 21)
+    batch = rh.make_relation_batch(B, fx.vocab.n_cat, 21)
     cond = get_cond(batch, tok, "relation", model_type="LayoutDM")
     cfg = rh.sampling_cfg("random", num_timesteps=25, relation_lambda=3e6, relation_mode="average", relation_tau=1.0, relation_num_update=3)
     res = {}

@@ -1,58 +1,39 @@
-"""The oracle's hand-derived restatement of the cond=relation logit adjustment (oracle.relation_update) against the
+"""The oracle's hand-derived restatement of the cond=relation logit adjustment (oracle.relation_update) against what the
 UNMODIFIED reference `update()` (logit_adjustment.py:88-126: autograd through _stochastic_convert and the 14 costs of
-models/clg/const.py) on synthetic relation batches built with the reference's own transforms (AddCanvasElement,
-AddRelationConstraints, data/util.py:106-170)."""
-import random
+models/clg/const.py) computed on synthetic relation batches built with the reference's own transforms (AddCanvasElement,
+AddRelationConstraints, data/util.py:106-170).  Batches, conditions and results are stored in tests/golden/ref_checks
+(tests/golden/make_ref_checks.py); the updated log-probs as the rows the update moved most plus a seeded sample."""
+import os
 
+import numpy as np
 import pytest
 import torch
 
 from oracle import layoutdm_oracle as O
-from oracle import ref_harness as rh
 
-pytestmark = pytest.mark.skipif(not rh.reference_available(), reason="reference not available")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_checks", "oracle_relation.npz")
 
 
-def make_relation_batch(B, n_cat, seed, edge_ratio=0.3):
-    rh._setup_path()
-    from trainer.data.util import AddCanvasElement, AddRelationConstraints
-    g = torch.Generator().manual_seed(seed)
-    add_c, add_r = AddCanvasElement(), AddRelationConstraints(seed=seed, edge_ratio=edge_ratio)
-    xs, ys, bs, ei, ea = [], [], [], [], []
-    off = 0
-    for b in range(B):
-        n = int(torch.randint(1, 26, (1,), generator=g)) if b else 25
-        class D:
-            pass
-        d = D()
-        d.x = torch.rand(n, 4, generator=g) * torch.tensor([1.0, 1.0, 0.6, 0.6]) + torch.tensor([0.0, 0.0, 0.02, 0.02])
-        d.y = torch.randint(0, n_cat, (n,), generator=g)
-        d.attr = {"has_canvas_element": torch.tensor(False)}
-        d = add_c(d)
-        d.attr["has_canvas_element"] = True
-        d = add_r(d)
-        xs.append(d.x); ys.append(d.y); bs.append(torch.full((n + 1,), b))
-        if d.edge_index.numel():
-            ei.append(d.edge_index + off); ea.append(d.edge_attr)
-        off += n + 1
-    batch = rh.FakeBatch(torch.cat(xs), torch.cat(ys), torch.cat(bs))
-    batch.edge_index = torch.cat(ei, dim=1) if ei else torch.zeros(2, 0, dtype=torch.long)
-    batch.edge_attr = torch.cat(ea) if ea else torch.zeros(0, dtype=torch.long)
-    batch.attr = {"has_canvas_element": True}
-    return batch
+@pytest.fixture(scope="module")
+def ref():
+    return np.load(GOLDEN)
+
+
+def tensor(z, key, dtype=torch.long):
+    return torch.from_numpy(z[key]).to(dtype)
+
+
+def adjacency(z, p, B):
+    return O.relation_adjacency(tensor(z, p + "edge_index"), tensor(z, p + "edge_attr"), tensor(z, p + "batch"), B, O.RICO25.n_elem + 1)
 
 
 @pytest.mark.parametrize("seed,t,lam,n_up", [(0, 50, 3e6, 3), (1, 10, 1e6, 1), (2, 9, 3e6, 3), (3, 99, 3e7, 5)])
-def test_relation_update_matches_reference_autograd(seed, t, lam, n_up):
-    torch.manual_seed(seed); random.seed(seed)
-    model, tok = rh.build_reference("rico25", T=100)
-    from trainer.helpers.task import get_cond
-    from trainer.models.categorical_diffusion.logit_adjustment import _stochastic_convert, update
+def test_relation_update_matches_reference_autograd(ref, seed, t, lam, n_up):
     vo = O.RICO25
     B = 5
-    batch = make_relation_batch(B, vo.n_cat, seed)
-    cond = get_cond(batch, tok, "relation", model_type="LayoutDM")
-    assert cond["seq"].shape == (B, vo.S) and "batch_w_canvas" in cond
+    p = f"update_{seed}_"
+    seq = tensor(ref, p + "seq")
+    assert seq.shape == (B, vo.S)
     # a log-prob tensor like the one the posterior hands over: log-softmax inside each attribute's group, log(1e-30) outside
     g = torch.Generator().manual_seed(seed + 7)
     lp = torch.full((B, vo.S, vo.C), O.LOG_EPS)
@@ -60,50 +41,42 @@ def test_relation_update_matches_reference_autograd(seed, t, lam, n_up):
         a = s % 5
         lo, n = vo.group_start(a), vo.group_n(a)
         lp[:, s, lo:lo + n] = torch.log_softmax(torch.randn(B, n, generator=g) * 2.0, dim=-1)
-    cfg = rh.sampling_cfg("random", relation_lambda=lam, relation_mode="average", relation_tau=1.0, relation_num_update=n_up)
-    want = update(t=t, cond=cond, model_log_prob=lp.permute(0, 2, 1).contiguous(), tokenizer=tok, sampling_cfg=cfg).permute(0, 2, 1)
+    x = lp.double()
+    assert np.allclose([float(x.sum()), float(x.abs().sum())], ref[p + "lp_checksum"], rtol=1e-9), "torch generator drifted from the stored inputs"
     centers = torch.stack([torch.as_tensor(c, dtype=torch.float32) for c in O.linear_centers(vo.n_bins)])
-    adj = O.relation_adjacency(batch.edge_index, batch.edge_attr, batch.batch, B, vo.n_elem + 1)
+    adj = adjacency(ref, p, B)
     # expected boxes first (the forward half)
-    bb_ref = _stochastic_convert(cond, lp.permute(0, 2, 1).contiguous(), tok)
-    p, bbox, valid = O.relation_bbox(lp, cond["seq"], centers, vo)
-    assert torch.allclose(bbox[valid], bb_ref, atol=1e-6)
-    got = O.relation_update(lp, cond["seq"], adj, centers, vo, t, lam, n_up)
-    moved = (want - lp).abs().max().item()
-    err = (got - want).abs().max().item()
-    print(f"seed {seed} t={t}: edges {batch.edge_index.shape[1]}, update moved log-probs by up to {moved:.3e}, |oracle - reference| {err:.3e}")
+    _, bbox, valid = O.relation_bbox(lp, seq, centers, vo)
+    assert torch.allclose(bbox[valid], tensor(ref, p + "bbox", torch.float32), atol=1e-6)
+    got = O.relation_update(lp, seq, adj, centers, vo, t, lam, n_up)
+    rows = (tensor(ref, p + "rows_b"), tensor(ref, p + "rows_s"))
+    want = tensor(ref, p + "want", torch.float32)
+    moved = float(ref[p + "moved"])
+    err = (got[rows] - want).abs().max().item()
+    print(f"seed {seed} t={t}: edges {ref[p + 'edge_index'].shape[1]}, update moved log-probs by up to {moved:.3e}, |oracle - reference| {err:.3e}")
     if t >= 10:
         assert moved > 1e-3, "test inputs do not exercise the update"
+        assert (got - lp).abs().max().item() > 1e-3
     assert err <= 2e-5 * max(1.0, moved)
 
 
-def test_relation_step_order_matches_reference_single_step():
+def test_relation_step_order_matches_reference_single_step(ref):
     """whole `_sample_single_step` (base.py:205-291) with cond=relation: strong mask -> update() -> PAD-disable -> draw, the
     reference (autograd update) against the oracle step with the hand-derived update; ids equal under the shared noise."""
-    import copy
-    torch.manual_seed(0); random.seed(0)
     vo, spec = O.RICO25, O.ModelSpec()
     sd = O.make_weights(vo, spec, seed=7, scale=2.0)
-    model, tok = rh.build_reference("rico25", T=100, state_dict=sd)
-    core = model.model.module
-    from trainer.helpers.task import get_cond
     B = 4
-    batch = make_relation_batch(B, vo.n_cat, 11)
-    cond = get_cond(batch, tok, "relation", model_type="LayoutDM")
+    seq, mask = tensor(ref, "step_seq"), tensor(ref, "step_mask", torch.bool)
     lam, n_up = 3e6, 3
-    cfg = rh.sampling_cfg("random", relation_lambda=lam, relation_mode="average", relation_tau=1.0, relation_num_update=n_up)
-    ocond = dict(seq=cond["seq"].clone(), mask=cond["mask"].clone(), type="relation", rel_lambda=lam, rel_num_update=n_up,
-                 rel_adj=O.relation_adjacency(batch.edge_index, batch.edge_attr, batch.batch, B, vo.n_elem + 1))
+    ocond = dict(seq=seq.clone(), mask=mask.clone(), type="relation", rel_lambda=lam, rel_num_update=n_up, rel_adj=adjacency(ref, "step_", B))
     orc = O.Oracle(vo, spec, sd)
     g = torch.Generator().manual_seed(3)
     for t in (60, 9):
-        x_t = torch.where(torch.rand(B, vo.S, generator=g) < 0.5, cond["seq"], torch.full_like(cond["seq"], vo.mask_id))
-        x_t = torch.where(cond["mask"], cond["seq"], x_t)
-        log_z = torch.log(torch.nn.functional.one_hot(x_t, vo.C).permute(0, 2, 1).float().clamp(min=1e-30))
+        x_t = torch.where(torch.rand(B, vo.S, generator=g) < 0.5, seq, torch.full_like(seq, vo.mask_id))
+        x_t = torch.where(mask, seq, x_t)
+        assert torch.equal(x_t, tensor(ref, f"step_{t}_x_t")), "torch generator drifted from the stored inputs"
         u = O.uniforms(5, t, 0, 0, B, vo.S, vo.C)
-        with rh.injected_multinomial(lambda i, rows, ncls: u.reshape(rows, ncls)):
-            out = core._sample_single_step(log_z=log_z, model_t=torch.full((B,), t), skip_step=0, sampling_cfg=cfg, cond=copy.copy(cond))
-        want = out.argmax(1)
+        want = tensor(ref, f"step_{t}_ids")
         lp, _ = orc.step_logprob(x_t, t, t, ocond)
         got = O.draw(lp, O.SamplingCfg(name="random"), u)
         assert torch.equal(got, want), f"t={t}: {(got != want).sum().item()} ids differ"
